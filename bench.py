@@ -70,7 +70,29 @@ def parse_args(argv=None):
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"], help="N>1: in-kernel peer-memory exchange (default) or host loop + NCCL all-reduce per batch")
     ap.add_argument("--ref-iterations", type=int, default=-1, help="NM iterations per reference-arm step (bounded sample); -1 = per-config default")
     ap.add_argument("--grid-poses", type=int, default=16384, help="C5: poses of the grid (16384 = the BASELINE figure)")
-    return ap.parse_args(argv)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float64), to compare two builds output for output")
+    args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, outputs):
+    """DIR/<name>.npy for every array a caller of the timed path receives, as float64.  The inputs are seeded, so two runs
+    with the same arguments can be compared file for file.  Past DUMP_LIMIT_BYTES in all, each array keeps a fixed, seeded,
+    sorted sample of its rows."""
+    outputs = {k: np.asarray(v, dtype=np.float64) for k, v in outputs.items()}
+    total = sum(a.nbytes for a in outputs.values())
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        if total > DUMP_LIMIT_BYTES and a.ndim > 0 and len(a) > 1:
+            keep = max(1, int(len(a) * DUMP_LIMIT_BYTES / total))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def start_poses(cfg, T_gt, count):
@@ -502,16 +524,22 @@ def main():
 
             nid = IG.score_poses(cost, grid, rank, world)
             mine = len(grid[rank::world])
-            return {"evals": len(grid) / world, "computed": mine, "batches": (mine + 7) // 8, "result": float(np.nanmin(nid))}
+            return {"evals": len(grid) / world, "computed": mine, "batches": (mine + 7) // 8, "result": float(np.nanmin(nid)), "outputs": {"grid_nid": nid}}
         ev = cm = bt = 0
         y = None
+        solves = []
         for T0 in starts:
-            _, r = VC.estimate_pose_on_costs([cost], T0, params, allreduce=ar)
+            T, r = VC.estimate_pose_on_costs([cost], T0, params, allreduce=ar)
             ev += r["num_evaluations"]
             cm += r["num_evaluations_computed"]
             bt += r["num_batches"]
             y = r["y"]
-        return {"evals": ev, "computed": cm, "batches": bt, "result": y, "iterations": r["num_iterations"]}
+            solves.append((T, r))
+        # per solve: the estimated T_camera_lidar, the Nelder-Mead minimiser and its cost, and the counts of the serial search
+        outputs = {"T_camera_lidar": [T for T, _ in solves], "nm_x": [r["x"] for _, r in solves], "nm_cost": [r["y"] for _, r in solves],
+                   "nm_converged": [r["converged"] for _, r in solves], "nm_iterations": [r["num_iterations"] for _, r in solves],
+                   "nm_evaluations": [r["num_evaluations"] for _, r in solves]}
+        return {"evals": ev, "computed": cm, "batches": bt, "result": y, "iterations": r["num_iterations"], "outputs": outputs}
 
     def e2e_step():
         if grid_mode:
@@ -563,6 +591,8 @@ def main():
         sampler.start()
     res, total_ms, wall, prof = timed(resident_step, args.steps, args.warmup, profile=True)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res[-1]["outputs"])
 
     evals_ref = sum(r["evals"] for r in res)      # what the serial reference would evaluate (this rank's bag / pose share)
     evals_cmp = sum(r["computed"] for r in res)   # poses actually scored
@@ -572,7 +602,7 @@ def main():
     mpoints = world * n_resident * evals_cmp / secs * 1e-6
 
     # ---- e2e: host buffers in, result out, every step -----------------------------------------------------------------------
-    e2e_res, e2e_ms, _, _ = timed(e2e_step, max(3, min(args.steps, 5)), 3, profile=False)
+    e2e_res, e2e_ms, _, _ = timed(e2e_step, args.steps, 3, profile=False)
     e2e_steps = len(e2e_res)
     e2e_evals = sum(r["evals"] for r in e2e_res)
     e2e_cmp = sum(r["computed"] for r in e2e_res)

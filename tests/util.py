@@ -1,7 +1,13 @@
 """Shared seeded test problems (inputs only; expected values always come from the oracle or golden files)."""
+import hashlib
+import json
+import os
+
 import numpy as np
 
 from direct_visual_lidar_calibration_b200 import synthetic as S
+
+REFERENCE_OUTPUTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_outputs.json")
 
 # model -> (intrinsics, distortion, (W, H))
 CAMERAS = {
@@ -44,3 +50,44 @@ def random_poses(T, count, seed=0, rot_deg=2.0, trans=0.1):
     for _ in range(count - 1):
         out.append(S.perturb(T, rng.uniform(-rot_deg, rot_deg, 3), rng.uniform(-trans, trans, 3)))
     return np.stack(out)
+
+
+def digest(a):
+    """SHA-256 of an array's shape and bits (floats as float64 with every NaN as one bit pattern, integers as int64): a
+    bit-exact comparison with an output too large to store.  Signed zeros and infinities count."""
+    a = np.asarray(a)
+    a = a.astype(np.float64) if a.dtype.kind == "f" else a.astype(np.int64)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a)
+    h = hashlib.sha256(repr(a.shape).encode())
+    h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def plain(x):
+    """numpy values -> JSON values (float64 round-trips exactly through json's repr of floats)."""
+    if isinstance(x, dict):
+        return {k: plain(v) for k, v in x.items()}
+    if isinstance(x, (list, tuple)):
+        return [plain(v) for v in x]
+    if isinstance(x, np.ndarray):
+        return plain(x.tolist())
+    if isinstance(x, (bool, np.bool_)):
+        return bool(x)
+    if isinstance(x, (int, np.integer)):
+        return int(x)
+    if isinstance(x, (float, np.floating)):
+        return float(x)
+    return x
+
+
+def reference_outputs():
+    """What the reference's own code returned on the seeded inputs of the reference comparisons
+    (tests/golden/make_reference_outputs.py)."""
+    with open(REFERENCE_OUTPUTS) as f:
+        return json.load(f)
+
+
+def same(a, b):
+    """Bit-for-bit equality of stored and computed values, NaN equal to NaN."""
+    return digest(a) == digest(b)
